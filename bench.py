@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 20 --warmup 5            # this repo's CUDA path on 1 GPU
     torchrun ... bench.py --gpus N ...                        # one rank per GPU, particle-sharded (weak scaling)
     python bench.py --impl reference ...                      # the reference algorithm on the host CPU cores
+    python bench.py ... --dump-outputs DIR                    # also save the last timed step's outputs as .npy
 
 A step is one ``Pips.forward(xys, rgbs, iters=6)`` over one synthetic batch:
   N=1   BASELINE configs[1]: B=4, S=8, 384x512, N=1024, iters=6, stride 8
@@ -208,19 +209,17 @@ def run_reference(args, rank, world):
 
     def step():
         with torch.no_grad():
-            po.forward(sd, xy, rg, iters=ITERS, stride=STRIDE, allpairs=True, faithful_dead_work=True)
+            return po.forward(sd, xy, rg, iters=ITERS, stride=STRIDE, allpairs=True, faithful_dead_work=True)
 
-    t0 = time.perf_counter(); step(); first = time.perf_counter() - t0
-    budget = 200.0
     steps, warm = args.steps, args.warmup
-    if first * (steps + warm) > budget:
-        steps = max(1, int(budget / first) - 1); warm = 1 if steps > 1 else 0
-    for _ in range(max(0, warm - 1)):
+    for _ in range(warm):
         step()
     t0 = time.perf_counter()
     for _ in range(steps):
-        step()
+        out = step()
     dt = (time.perf_counter() - t0) / steps
+    if args.dump_outputs:
+        dump_outputs(out, args.dump_outputs)
     val = bs * S * ns * ITERS / dt
     sample = f"B={bs} of {B}, N={ns} of {N_PER_GPU}, iters={ITERS}, incl. fnet, all-pairs volume + dense heat-map as the reference computes them"
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": steps, "warmup": warm,
@@ -249,6 +248,25 @@ def cpu_baseline_leg():
         dt = (time.perf_counter() - t0) / reps
     return {"value": bs * S * ns * ITERS / dt, "unit": UNIT, "cores": cores, "kind": "port",
             "sample": f"B={bs} of {B}, N={ns} of {N_PER_GPU}, iters={ITERS}, {reps} forwards incl. fnet, reference algorithm (all-pairs volume + dense heat-map)"}
+
+
+DUMP_BYTES = 63 * 10**6                   # array data; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out, directory: str) -> None:
+    """What ``Pips.forward`` handed its caller, as float32 ``<name>.npy`` in ``directory``: coord_predictions
+    (iters,B,S,N,2), coord_predictions2 (iters+4,B,S,N,2) and vis_e (B,S,N).  When they hold more than DUMP_BYTES,
+    every k-th particle is written (the smallest k that fits), the same particles in every array."""
+    import numpy as np
+    preds, preds2, vis_e, _ = out
+    arrays = {"coord_predictions": (torch.stack(preds), 3), "coord_predictions2": (torch.stack(preds2), 3), "vis_e": (vis_e, 2)}
+    n = vis_e.shape[2]
+    per_particle = sum(a.numel() // n * 4 for a, _ in arrays.values())
+    every = -(-n // max(1, DUMP_BYTES // per_particle))
+    os.makedirs(directory, exist_ok=True)
+    for name, (a, dim) in arrays.items():
+        keep = torch.arange(0, n, every, device=a.device)
+        np.save(os.path.join(directory, name + ".npy"), a.index_select(dim, keep).float().cpu().numpy())
 
 
 def _stats(per_ms: list) -> dict:
@@ -414,16 +432,17 @@ def run_ours(args, rank, world, local_rank):
             return out[0][-1].cpu(), out[2].cpu()
 
     def timed(step, k):
-        """k steps, L2 flushed before each; returns (total seconds, [ms per step]) from CUDA events on this stream."""
-        evs = []
+        """k steps, L2 flushed before each; returns (total seconds, [ms per step], output of the last step) from CUDA
+        events on this stream."""
+        evs, out = [], None
         for _ in range(k):
             flush.zero_()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record(); step(); e1.record()
+            e0.record(); out = step(); e1.record()
             evs.append((e0, e1))
         torch.cuda.synchronize()
         per = [a.elapsed_time(b) for a, b in evs]
-        return sum(per) / 1e3, per
+        return sum(per) / 1e3, per, out
 
     # sharded runs: the particle shares become speed-weighted after the 5th forward (pips_b200/sharding.py::_Balance) and the
     # next forward re-captures its CUDA graph at the new share -- all of that belongs to the warm-up
@@ -437,9 +456,11 @@ def run_ours(args, rank, world, local_rank):
         step_device()
     barrier()
     sampler.mark()
-    t_dev, per_dev = timed(step_device, args.steps)
+    t_dev, per_dev, last = timed(step_device, args.steps)
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last, args.dump_outputs)
     if world > 1:
         all_clocks = [None] * world
         dist.all_gather_object(all_clocks, clocks)
@@ -450,7 +471,7 @@ def run_ours(args, rank, world, local_rank):
     launches = (model.engine.launches + (encoder_fast.LAUNCHES[0] if model.fnet_mode == 'tc' else 0)) * args.steps
     step_host()
     barrier()
-    t_e2e, per_e2e = timed(step_host, args.steps)
+    t_e2e, per_e2e, _ = timed(step_host, args.steps)
     barrier()
     if world > 1:
         t = torch.tensor([t_dev, t_e2e], device=dev, dtype=torch.float64)
@@ -632,7 +653,11 @@ def main():
     ap.add_argument("--no-eager", action="store_true", help="skip the eager-torch restatement of the reference on this GPU")
     ap.add_argument("--no-extra", action="store_true", help="skip the other BASELINE configurations (n4096_1gpu, cfg1/4/5, strong_cfg3, cfg4_sharded)")
     ap.add_argument("--particles", type=int, default=0, help="particles per GPU (default 1024 = BASELINE cfg2; 4096 = cfg3 on one GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as float32 DIR/<name>.npy "
+                                                            "(inputs are seeded: runs with the same arguments are comparable)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     if args.particles > 0:

@@ -1,6 +1,8 @@
-"""Generate golden vectors from the UNMODIFIED reference (run in the build container only).
+"""Generate golden vectors from the UNMODIFIED reference (a checkout of aharley/pips).
 
-    python tests/golden/make_golden.py          # needs /root/reference
+    python tests/golden/make_golden.py --reference DIR [--cfg2 | --cfg4 | --demo | --nets-layout]
+
+The tests import only the case definitions and input generators below; they never need the reference.
 
 The reference (aharley/pips, nets/pips.py) is imported as-is; the only shim is
 ``torch.Tensor.cuda = identity`` because nets/pips.py:429 calls ``.cuda()`` on a
@@ -18,7 +20,6 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, "/root/reference")
 
 from oracle import pips_oracle as po  # noqa: E402
 
@@ -216,10 +217,10 @@ def main_cfg4():
     print("wrote", os.path.join(HERE, "reference_cfg4.npz"), os.path.getsize(os.path.join(HERE, "reference_cfg4.npz")), "bytes")
 
 
-# BASELINE cfg 1 on the REAL demo clip: /root/reference/demo_images/000100-000107.jpg decoded with PIL, the recipe of
+# BASELINE cfg 1 on the REAL demo clip: the reference's demo_images/000100-000107.jpg decoded with PIL, the recipe of
 # demo.py:21-41 (float, bilinear resize to 360 x 640, 16 x 16 query grid with an 8 px margin, model(xy, rgbs, iters=6)),
 # stride 4 as demo.py:114.  The eight JPEG files (320 KB) are stored inside the fixture together with the SHA-256 of the
-# decoded pixels, so that the test on the GPU box -- where /root/reference does not exist -- feeds the same bytes.
+# decoded pixels, so that the test feeds the same bytes without a reference checkout.
 DEMO_CASE = dict(B=1, H=360, W=640, N=256, stride=4, iters=6, head_scale=0.05, seed=11)
 DEMO_FRAMES = list(range(100, 108))
 
@@ -245,14 +246,14 @@ def demo_inputs(rgbs):
     return rgbs, torch.stack([gx, gy], dim=-1)
 
 
-def main_demo():
+def main_demo(reference):
     import hashlib
     torch.Tensor.cuda = lambda self, *a, **k: self
     from nets.pips import Pips  # the reference, unmodified
 
     torch.set_num_threads(min(16, os.cpu_count() or 1))
     c = DEMO_CASE
-    blobs = [open(f"/root/reference/demo_images/{i:06d}.jpg", "rb").read() for i in DEMO_FRAMES]
+    blobs = [open(os.path.join(reference, "demo_images", f"{i:06d}.jpg"), "rb").read() for i in DEMO_FRAMES]
     raw = demo_decode(blobs)
     rgbs, xy = demo_inputs(raw)
     sd = po.init_state_dict(seed=c["seed"], head_scale=c["head_scale"])
@@ -269,12 +270,29 @@ def main_demo():
     print("wrote", os.path.join(HERE, "reference_demo.npz"), os.path.getsize(os.path.join(HERE, "reference_demo.npz")), "bytes")
 
 
+# The module files of the reference's `nets` package (paths relative to the checkout, no contents): the zero-edit shim
+# test rebuilds the package from empty stand-ins at these paths to check that shim/nets/pips.py shadows nets.pips only.
+def main_nets_layout(reference):
+    import json
+    mods = sorted(os.path.relpath(os.path.join(d, f), reference).replace(os.sep, "/")
+                  for d, _, files in os.walk(os.path.join(reference, "nets")) for f in files if f.endswith(".py"))
+    with open(os.path.join(HERE, "reference_nets_layout.json"), "w") as f:
+        json.dump(mods, f, indent=1)
+    print("wrote", os.path.join(HERE, "reference_nets_layout.json"), mods)
+
+
 if __name__ == "__main__":
+    if "--reference" not in sys.argv[:-1]:
+        sys.exit(__doc__.split("\n\n")[1])
+    REFERENCE = os.path.abspath(sys.argv[sys.argv.index("--reference") + 1])
+    sys.path.insert(0, REFERENCE)
     if "--cfg2" in sys.argv:
         main_cfg2()
     elif "--cfg4" in sys.argv:
         main_cfg4()
     elif "--demo" in sys.argv:
-        main_demo()
+        main_demo(REFERENCE)
+    elif "--nets-layout" in sys.argv:
+        main_nets_layout(REFERENCE)
     else:
         main()

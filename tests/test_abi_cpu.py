@@ -148,17 +148,26 @@ def test_plain_c_consumer_links_and_struct_layouts_match(tmp_path):
     assert int(sizes["pips_problem"]) == ctypes.sizeof(L.Problem)
 
 
-def test_zero_edit_shim_serves_nets_pips():
-    """shim/ before the reference on sys.path: `from nets.pips import Pips` (demo.py:9) is pips_b200.Pips, other modules
-    of the reference's `nets` package still resolve to the reference checkout (when it is present)."""
+def test_zero_edit_shim_serves_nets_pips(tmp_path):
+    """shim/ before the reference on sys.path: `from nets.pips import Pips` (demo.py:9) is pips_b200.Pips, every other
+    module of the reference's `nets` package still resolves to the reference checkout.  The checkout is stood in for by
+    empty modules at the paths recorded from it (tests/golden/reference_nets_layout.json); its nets/pips.py fails if imported."""
+    import json
     import subprocess
     import sys
-    ref = "/root/reference"
-    code = ("import sys; from nets.pips import Pips; import pips_b200; assert Pips is pips_b200.Pips; "
-            "m = Pips(S=8, stride=4); assert len(m.state_dict()) == 200; print('shim ok')")
-    if os.path.isdir(ref):
-        code += "; import nets.raft_core.util as u; assert u.__file__.startswith('/root/reference'); print('reference nets.* still visible')"
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, "shim"), ROOT] + ([ref] if os.path.isdir(ref) else [])))
+    with open(os.path.join(ROOT, "tests", "golden", "reference_nets_layout.json")) as f:
+        layout = json.load(f)
+    assert "nets/pips.py" in layout and "nets/raft_core/util.py" in layout
+    ref = tmp_path / "reference"
+    for rel in layout:
+        (ref / rel).parent.mkdir(parents=True, exist_ok=True)
+        (ref / rel).write_text("raise ImportError('the reference nets.pips shadowed the shim')\n" if rel == "nets/pips.py" else "")
+    others = [rel[:-3].replace("/", ".").removesuffix(".__init__") for rel in layout if rel != "nets/pips.py"]
+    code = ("import importlib; from nets.pips import Pips; import pips_b200; assert Pips is pips_b200.Pips; "
+            "m = Pips(S=8, stride=4); assert len(m.state_dict()) == 200; print('shim ok'); "
+            f"assert all(importlib.import_module(n).__file__.startswith({str(ref)!r}) for n in {others!r}); "
+            "print('reference nets.* still visible')")
+    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, "shim"), ROOT, str(ref)]))
     out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, timeout=300)
     assert out.returncode == 0, out.stderr[-2000:]
-    assert "shim ok" in out.stdout
+    assert "shim ok" in out.stdout and "reference nets.* still visible" in out.stdout
