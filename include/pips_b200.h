@@ -148,6 +148,32 @@ size_t pips_heatmap_scratch_floats(int frames, int n_sel, int H8, int W8);
 int pips_heatmap(const void* const* lvl, int feat_dtype, int B, int S, int N, int H8, int W8, const float* ffeats,
                  const int* sel, const int* slot, int n_sel, float* scratch, float* out, size_t out_frame_stride, void* stream);
 
+/* ---- score-map loss of a supervised evaluation call (nets/pips.py:58-90 score_map_loss with :14-37 balanced_ce_loss,
+ * on the score maps of :502-511), without the dense (B,S,I,N,H8,W8) score maps.  Always bf16x3 on tcgen05, whatever
+ * the mixer precision.  Order per forward: pips_score_grid once after the pyramid, pips_score_loss once per iteration
+ * before pips_refine_iter (it reads the ffeats the iteration starts from), pips_score_loss_finalize once at the end.
+ *
+ * Replaces nets/pips.py:504-511 for the loss: bilinear interpolation is linear, so every score map is <f, Gr> with
+ *   Gr = sum_l interpolate(lvl_f32[l] -> H8 x W8, bilinear, align_corners=True) / sqrt(128)
+ * grid: (2, frames, Ppad, 128) bf16 -- the hi plane, then the lo plane (Gr ~= hi + lo); Ppad = H8*W8 rounded up to
+ * PIPS_SCORE_TILE, padding rows zero. */
+enum { PIPS_SCORE_TILE = 256 };
+int pips_score_grid(const float* const* lvl_f32, int frames, int H8, int W8, void* grid, void* stream);
+/* floats of the `partial` buffer for rows = B*S*n_total tracks and `iters` iterations (0 for an empty problem) */
+size_t pips_score_loss_scratch_floats(int rows, int iters, int H8, int W8);
+/* nets/pips.py:58-90 per iteration, for particles [n_offset, n_offset + N) of n_total: the GEMM of the score maps with
+ * an epilogue that writes, per (track, 128-pixel block), the sum of softplus(fcp) over the block's pixels other than the
+ * target, and fcp at the target.  ffeats (B*N, S, 128) fp32 is the loop state of this call's particles; target
+ * (B, S, n_total) int32 holds y*W8 + x of the rounded ground truth (stride-scaled), or -1 for a track the loss excludes
+ * (outside the map, valids == 0 or vis_g == 0).  Every partial depends only on its (track, pixel block): chunking the
+ * particles over several calls gives identical bits. */
+int pips_score_loss(const void* grid, int B, int S, int N, int H8, int W8, const float* ffeats, const int* target,
+                    int n_offset, int n_total, int iter, int iters, float* partial, void* stream);
+/* nets/pips.py:14-37 + :58-90 (masked means): reduces the partials of all iterations in fp64 in a fixed order, counts
+ * the kept tracks K from target, and writes ce = sum_pos / (1e-6 + K*I) + sum_neg / (1e-6 + K*I*(H8*W8 - 1)) (fp32,
+ * 0 when K = 0) to *ce. */
+int pips_score_loss_finalize(const int* target, int rows, int iters, int H8, int W8, float* partial, float* ce, void* stream);
+
 /* v -> (hi, lo) bf16 with hi = rn(v), lo = rn(v - hi); lo may be NULL.  Used to pack weights. */
 int pips_split_bf16(const float* src, void* hi, void* lo, size_t n, void* stream);
 

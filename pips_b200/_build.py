@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "lib", "obj")
 LIB = os.path.join(HERE, "lib", "libpips_b200.so")
-SOURCES = ["abi.cu", "pyramid.cu", "corr_gather.cu", "mixer_simt.cu", "tokenmix_tc.cu", "gemm_tc.cu", "gemm_tc2.cu", "conv_tc.cu", "conv_rows.cu", "encoder_ops.cu", "heatmap.cu", "peer.cu"]
+SOURCES = ["abi.cu", "pyramid.cu", "corr_gather.cu", "mixer_simt.cu", "tokenmix_tc.cu", "gemm_tc.cu", "gemm_tc2.cu", "conv_tc.cu", "conv_rows.cu", "encoder_ops.cu", "heatmap.cu", "score_loss.cu", "peer.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v", "--expt-relaxed-constexpr"]
 

@@ -22,6 +22,7 @@ HEAD_PAD = 1280
 FEAT_F32, FEAT_BF16 = 0, 1
 PREC_F32, PREC_BF16X3, PREC_BF16 = 0, 1, 2
 EPI_BIAS, EPI_BIAS_GELU, EPI_BIAS_RESID = 0, 1, 2
+SCORE_TILE = 256           # PIPS_SCORE_TILE: the score-loss grid's pixel rows are padded to a multiple of this
 
 PRECISIONS = {"fp32": PREC_F32, "bf16x3": PREC_BF16X3, "bf16": PREC_BF16}
 FEAT_DTYPES = {"fp32": FEAT_F32, "bf16": FEAT_BF16}
@@ -86,6 +87,10 @@ _SIGNATURES = {
     "pips_ln_pool": (_i, [_p, _i, _p, _p, _p, _p, _p, _p]),
     "pips_update": (_i, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _f, _i, _i, _i, _p]),
     "pips_vis_head": (_i, [_p, _p, _p, _p, _i, _i, _i, _p]),
+    "pips_score_grid": (_i, [C.POINTER(_p), _i, _i, _i, _p, _p]),
+    "pips_score_loss_scratch_floats": (C.c_size_t, [_i, _i, _i, _i]),
+    "pips_score_loss": (_i, [_p, _i, _i, _i, _i, _i, _p, _p, _i, _i, _i, _i, _p, _p]),
+    "pips_score_loss_finalize": (_i, [_p, _i, _i, _i, _i, _p, _p, _p]),
     "pips_split_bf16": (_i, [_p, _p, _p, C.c_size_t, _p]),
     "pips_inorm_stats": (_i, [_p, _i, _i, _i, _p, _i, _p, _p]),
     "pips_inorm_apply": (_i, [_p, _p, _p, _p, _i, _i, _p, _p, _i, _i, _i, _i, _p]),

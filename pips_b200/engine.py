@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-from typing import Dict, Optional, Tuple
+from typing import Dict, Optional
 
 import torch
 
@@ -276,15 +276,19 @@ class RefineEngine:
     # ------------------------------------------------------------------ the loop
     def _enqueue(self, lib, wc, pyr: Pyramid, ws: Workspace, fmaps2d, c, c0, ffeat, ffeats, feat_init, out, vis,
                  B, S, nc, H8, W8, iters, stride, on_iter=None, build_pyramid=True, frame_base=None, T=0,
-                 heat=None, peer=None, peer_n0=0) -> int:
+                 heat=None, score_loss=None, peer=None, peer_n0=0) -> int:
         """Enqueue every launch of one forward for ``nc`` particles on the current stream: pyramid, initial
-        features, ``iters`` refinement iterations, visibility head.  Returns the number of kernels launched."""
+        features, ``iters`` refinement iterations, visibility head.  Returns the number of kernels launched.
+        ``score_loss`` (``_ScoreLoss``): also the score-map loss of these particles (nets/pips.py:58-90)."""
         st = self._stream()
         launches = 0
         if build_pyramid:
             with nvtx_range("pips/pyramid"):
                 pyr.build(fmaps2d, st)
             launches += 4
+            if score_loss is not None:
+                L.check(lib.pips_score_grid(pyr.f32_ptrs, B * S, H8, W8, L.ptr(score_loss.grid), st), "pips_score_grid")
+                launches += 1
         c0.copy_(c)
         if feat_init is None:
             L.check(lib.pips_init_gather(L.ptr(pyr.f32[0]), B, S, nc, H8, W8, L.ptr(c), L.ptr(frame_base), T, L.ptr(ffeat),
@@ -319,6 +323,11 @@ class RefineEngine:
                                          sel.numel(), L.ptr(scratch), L.ptr(fcps[0, 0, it]),
                                          fcps.stride(1), st), "pips_heatmap")
                 launches += 1 + (sel.numel() + 31) // 32
+            if score_loss is not None:              # nets/pips.py:502-511 + :58-90: loss terms of the starting state
+                sl = score_loss
+                L.check(lib.pips_score_loss(L.ptr(sl.grid), B, S, nc, H8, W8, L.ptr(ffeats), L.ptr(sl.target), peer_n0,
+                                            sl.n_total, it, iters, L.ptr(sl.partial), st), "pips_score_loss")
+                launches += 1
             with nvtx_range(f"pips/iter{it}"):
                 L.check(lib.pips_refine_iter(C.byref(prob), C.byref(wc), C.byref(ws.c), L.ptr(out[it]), st), "pips_refine_iter")
             launches += 1 + (1 + 3 * L.DEPTH + 2) + 1
@@ -326,12 +335,16 @@ class RefineEngine:
                 on_iter(it, out[it])
         with nvtx_range("pips/vis_head"):
             L.check(lib.pips_vis_head(L.ptr(ffeats), wc.vis_w, wc.vis_b, L.ptr(vis), B, S, nc, st), "pips_vis_head")
+        if score_loss is not None and peer_n0 + nc == score_loss.n_total:      # the last chunk: reduce all partials
+            L.check(lib.pips_score_loss_finalize(L.ptr(score_loss.target), score_loss.target.numel(), iters, H8, W8,
+                                                 L.ptr(score_loss.partial), L.ptr(score_loss.ce), st), "pips_score_loss_finalize")
+            launches += 2
         return launches + 1
 
     def refine(self, module, fmaps: torch.Tensor, coords: torch.Tensor, feat_init: Optional[torch.Tensor],
                iters: int, stride: float, on_iter=None, frame_base: Optional[torch.Tensor] = None,
                reuse_pyramid: bool = False, heat_sel: Optional[torch.Tensor] = None,
-               heat_out: Optional[torch.Tensor] = None, peer=None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+               heat_out: Optional[torch.Tensor] = None, peer=None, score_target: Optional[torch.Tensor] = None):
         """fmaps (B,S,128,H8,W8) fp32, coords (B,S,N,2) fp32 in feature-map pixels.
         Returns preds (iters,B,S,N,2) in input pixels, vis_e (B,S,N) logits, ffeat (B,N,128).
         ``on_iter(it, coords_px)`` (optional) is called once per iteration when the particles fit one
@@ -342,7 +355,10 @@ class RefineEngine:
         ``heat_sel`` (n_sel,) particle indices + ``heat_out`` (B,S,iters,n_sel,H8,W8) fp32: also write the score maps
         of those particles (nets/pips.py:504-511) at the start of every iteration (eager launches, no graph).
         ``peer`` (pips_b200.peer.PeerPlan): this call refines one rank's slice of a particle-sharded run; the update
-        kernel also stores every iteration's prediction into all ranks' slabs (the caller runs the barriers)."""
+        kernel also stores every iteration's prediction into all ranks' slabs (the caller runs the barriers).
+        ``score_target`` (B,S,N) int32 (pips_b200.supervised.score_targets): also compute the score-map loss
+        (nets/pips.py:58-90) of the run; the result is then (preds, vis_e, ffeat, ce) with ce a 0-dim fp32 tensor.  The
+        score maps are never stored, and preds / vis_e / ffeat are those of the same call without it."""
         lib = L.load()
         B, T, Cc, H8, W8 = fmaps.shape
         S = coords.shape[1]
@@ -366,20 +382,27 @@ class RefineEngine:
             assert n_sel > 0 and int(heat_sel.min()) >= 0 and int(heat_sel.max()) < N, "heat_sel out of range"
             assert heat_out is not None and tuple(heat_out.shape) == (B, S, iters, n_sel, H8, W8) \
                 and heat_out.dtype == torch.float32 and heat_out.is_contiguous() and heat_out.device == dev
+        score = score_target is not None
+        if score:
+            if frame_base is not None or heat_sel is not None or peer is not None or iters <= 0:
+                raise L.PipsCudaError("pips_b200: the score-map loss needs iters > 0 and a plain, unsharded forward")
+            assert tuple(score_target.shape) == (B, S, N) and score_target.dtype == torch.int32 \
+                and score_target.device == dev, "score_target must be (B,S,N) int32 on the device of fmaps"
         if N <= chunk and self.use_graph and iters > 0 and frame_base is None and heat_sel is None:
             plan = self._plan(w, B, S, N, H8, W8, iters, float(stride), feat_init is not None, dev,
-                              nhwc=not fmaps2d.is_contiguous(), peer=peer)
-            preds, vis, ffeat = plan.run(fmaps2d, coords, feat_init)
+                              nhwc=not fmaps2d.is_contiguous(), peer=peer, score=score)
+            preds, vis, ffeat, ce = plan.run(fmaps2d, coords, feat_init, score_target)
             self.launches = plan.launches
             if on_iter is not None:
                 for it in range(iters):
                     on_iter(it, preds[it])
-            return preds, vis, ffeat
+            return (preds, vis, ffeat, ce) if score else (preds, vis, ffeat)
 
         pyr = self.pyramid(B * T, H8, W8, dev)
         preds = torch.empty(iters, B, S, N, 2, dtype=torch.float32, device=dev)
         vis = torch.empty(B, S, N, dtype=torch.float32, device=dev)
         ffeat_out = torch.empty(B, N, LATENT, dtype=torch.float32, device=dev)
+        sl = _ScoreLoss(B, S, N, H8, W8, iters, dev, score_target.contiguous()) if score else None
         self.launches = 0
         for n0 in range(0, N, chunk):
             n1 = min(N, n0 + chunk)
@@ -402,20 +425,23 @@ class RefineEngine:
             self.launches += self._enqueue(lib, w.c, pyr, ws, fmaps2d, c, c0, ffeat, ffeats, fi, out, v, B, S, nc, H8, W8,
                                            iters, stride, on_iter if whole else None,
                                            build_pyramid=(n0 == 0 and not reuse_pyramid), frame_base=fb, T=T, heat=heat,
-                                           peer=peer, peer_n0=n0)
+                                           score_loss=sl, peer=peer, peer_n0=n0)
             if not whole:
                 preds[:, :, :, n0:n1] = out
                 vis[:, :, n0:n1] = v
             ffeat_out[:, n0:n1] = ffeat.reshape(B, nc, LATENT)
+        if score:
+            return preds, vis, ffeat_out, sl.ce.reshape(())
         return preds, vis, ffeat_out
 
-    def _plan(self, w: PackedWeights, B, S, N, H8, W8, iters, stride, has_feat, dev, nhwc=False, peer=None) -> "_GraphPlan":
-        key = (id(w), B, S, N, H8, W8, iters, stride, has_feat, str(dev), nhwc, None if peer is None else peer.key)
+    def _plan(self, w: PackedWeights, B, S, N, H8, W8, iters, stride, has_feat, dev, nhwc=False, peer=None,
+              score=False) -> "_GraphPlan":
+        key = (id(w), B, S, N, H8, W8, iters, stride, has_feat, str(dev), nhwc, None if peer is None else peer.key, score)
         plan = self._plans.get(key)
         if plan is None:
             while len(self._plans) >= 2:                          # each plan owns a full workspace
                 self._plans.pop(next(iter(self._plans)))
-            plan = _GraphPlan(self, w, B, S, N, H8, W8, iters, stride, has_feat, dev, nhwc, peer)
+            plan = _GraphPlan(self, w, B, S, N, H8, W8, iters, stride, has_feat, dev, nhwc, peer, score)
             self._plans[key] = plan
         else:
             self._plans[key] = self._plans.pop(key)               # LRU order
@@ -491,13 +517,28 @@ class RefineEngine:
         return {k: [a.elapsed_time(b) for a, b in v] for k, v in rec.items()}, dict(B=B, S=S, N=N, M=M)
 
 
+class _ScoreLoss:
+    """Device buffers of the score-map loss of one forward: ``target`` (B,S,N) int32 (pixel index or -1), the bf16
+    (hi, lo) grid ``Gr`` of pips_score_grid, the per-(track, pixel block) ``partial`` sums and the ``ce`` scalar."""
+
+    def __init__(self, B, S, N, H8, W8, iters, dev, target=None):
+        lib = L.load()
+        ppad = _round_up(H8 * W8, L.SCORE_TILE)
+        self.n_total = N
+        self.target = target if target is not None else torch.full((B, S, N), -1, dtype=torch.int32, device=dev)
+        self.grid = torch.empty(2, B * S, ppad, LATENT, dtype=torch.bfloat16, device=dev)
+        self.partial = torch.empty(lib.pips_score_loss_scratch_floats(B * S * N, iters, H8, W8), dtype=torch.float32,
+                                   device=dev)
+        self.ce = torch.zeros(1, dtype=torch.float32, device=dev)
+
+
 class _GraphPlan:
     """One captured CUDA graph of a whole forward (pyramid .. vis head) for a fixed problem signature,
     with its own static buffers; replayed with new inputs copied in.  ~250 launches per forward collapse
     into one graph launch, which is what matters for small problems (demo / chained windows)."""
 
     def __init__(self, eng: RefineEngine, w: PackedWeights, B, S, N, H8, W8, iters, stride, has_feat, dev, nhwc=False,
-                 peer=None):
+                 peer=None, score=False):
         lib = L.load()
         self.w = w
         self.peer = peer                              # the captured update kernels store into these slabs
@@ -515,6 +556,7 @@ class _GraphPlan:
         self.preds = torch.zeros(iters, B, S, N, 2, **f32)
         self.vis = torch.zeros(B, S, N, **f32)
         self.shape = (B, N)
+        self.score = _ScoreLoss(B, S, N, H8, W8, iters, dev) if score else None      # static target / partials / ce
         eng.times(dev)
 
         self.nhwc = nhwc
@@ -522,7 +564,7 @@ class _GraphPlan:
         def enqueue():
             return eng._enqueue(lib, w.c, self.pyr, self.ws, self.fmaps_nhwc if nhwc else self.fmaps_nchw, self.c, self.c0,
                                 self.ffeat, self.ffeats, self.feat_in, self.preds, self.vis, B, S, N, H8, W8, iters, stride,
-                                peer=peer)
+                                score_loss=self.score, peer=peer)
 
         side = torch.cuda.Stream(device=dev)
         side.wait_stream(torch.cuda.current_stream(dev))
@@ -534,11 +576,14 @@ class _GraphPlan:
         with torch.cuda.graph(self.graph):
             enqueue()
 
-    def run(self, fmaps2d, coords, feat_init):
+    def run(self, fmaps2d, coords, feat_init, score_target=None):
         B, N = self.shape
         (self.fmaps_nhwc if self.nhwc else self.fmaps_nchw).copy_(fmaps2d)
         self.c.copy_(coords)
         if self.feat_in is not None:
             self.feat_in.copy_(feat_init)
+        if self.score is not None:
+            self.score.target.copy_(score_target)
         self.graph.replay()
-        return self.preds.clone(), self.vis.clone(), self.ffeat.reshape(B, N, LATENT).clone()
+        ce = self.score.ce.reshape(()).clone() if self.score is not None else None
+        return self.preds.clone(), self.vis.clone(), self.ffeat.reshape(B, N, LATENT).clone(), ce

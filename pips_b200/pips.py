@@ -15,7 +15,12 @@ Extra, optional knobs (keyword-only; the reference signature is unchanged):
               operands, element-wise stages fused, channels-last), 'fast' (cuDNN TF32 tensor-core
               convolutions over hi/lo-split operands instead), 'x3' (the same cuDNN convolutions through
               eager torch ops) or 'plain' (strict fp32 cuDNN)
-Environment overrides: PIPS_B200_PRECISION, PIPS_B200_FEAT, PIPS_B200_FNET.
+  supervised  'torch' (default) or 'cuda': where a supervised evaluation call runs -- ground truth given, is_train=False,
+              gradients off, no summary to save, CUDA inputs, not particle-sharded, not an nn.DataParallel replica.
+              'cuda' runs it on the inference kernels and computes the score-map loss without the dense score maps
+              (pips_b200/supervised.py; that loss is always bf16x3 on the tensor cores, whatever ``precision`` says).
+              Every other supervised or training call stays on the torch path (torch_path.py).
+Environment overrides: PIPS_B200_PRECISION, PIPS_B200_FEAT, PIPS_B200_FNET, PIPS_B200_SUPERVISED.
 """
 from __future__ import annotations
 
@@ -91,7 +96,7 @@ def _conv_math(allow_tf32: bool):
 
 class Pips(nn.Module):
     def __init__(self, S=8, stride=8, *, precision: Optional[str] = None, feat_dtype: Optional[str] = None,
-                 fnet_mode: Optional[str] = None, max_seqs: int = 32768):
+                 fnet_mode: Optional[str] = None, max_seqs: int = 32768, supervised: Optional[str] = None):
         super().__init__()
         self.S = S
         self.stride = stride
@@ -116,6 +121,10 @@ class Pips(nn.Module):
             raise ValueError("fnet_mode must be 'tc' (tcgen05 implicit-GEMM convolutions, bf16x3), 'fast' (cuDNN 3xTF32 "
                              "convolutions, channels-last, fused element-wise kernels), 'x3' (3xTF32 convolutions through "
                              "eager torch ops) or 'plain' (strict fp32 cuDNN)")
+        self.supervised = supervised or os.environ.get("PIPS_B200_SUPERVISED", "torch")
+        if self.supervised not in ("torch", "cuda"):
+            raise ValueError("supervised must be 'torch' (supervised calls on the differentiable torch path) or 'cuda' "
+                             "(evaluation calls on the CUDA kernels, score-map loss without dense score maps)")
 
     # ------------------------------------------------------------------ configuration
     @property
@@ -186,7 +195,14 @@ class Pips(nn.Module):
         assert (D == 2)
         B, S, C, H, W = rgbs.shape
 
-        slow = trajs_g is not None or is_train or (sw is not None and getattr(sw, "save_this", False))
+        save = sw is not None and getattr(sw, "save_this", False)
+        if (trajs_g is not None and self.supervised == "cuda" and not is_train and not torch.is_grad_enabled() and not save
+                and rgbs.is_cuda and self._shard is None and not getattr(self, "_is_replica", False)):
+            if N == 0:
+                raise RuntimeError("pips_b200.Pips: no particles (xys has N = 0); the reference raises here as well")
+            from .supervised import forward_cuda
+            return forward_cuda(self, xys, rgbs, coords_init, feat_init, iters, trajs_g, vis_g, valids, return_feat)
+        slow = trajs_g is not None or is_train or save
         if slow:
             from .torch_path import forward_torch
             return forward_torch(self, xys, rgbs, coords_init=coords_init, feat_init=feat_init, iters=iters,
@@ -235,6 +251,15 @@ class Pips(nn.Module):
 
     def refine(self, xys, fmaps, coords_init=None, feat_init=None, iters=3, return_feat=False):
         """Everything after fnet (nets/pips.py:450-611) given precomputed feature maps."""
+        coord_predictions, coord_predictions2, vis_e, ffeat, _ = self._refine(xys, fmaps, coords_init, feat_init, iters)
+        losses = None
+        if return_feat:
+            return coord_predictions, coord_predictions2, vis_e, ffeat, losses
+        return coord_predictions, coord_predictions2, vis_e, losses
+
+    def _refine(self, xys, fmaps, coords_init, feat_init, iters, score_target=None):
+        """refine() as (coord_predictions, coord_predictions2, vis_e, ffeat, ce); ``score_target`` (B,S,N) int32
+        (supervised.score_targets) also computes the score-map loss ``ce``, else ce is None."""
         B, N, _ = xys.shape
         S = fmaps.shape[1]
         stride = float(self.stride)
@@ -246,7 +271,11 @@ class Pips(nn.Module):
         if feat_init is not None:
             feat_init = feat_init.detach().float()
 
-        if self._shard is None or self._shard[1] == 1:
+        ce = None
+        if score_target is not None:
+            preds, vis_e, ffeat, ce = self._engine.refine(self, fmaps.float(), coords, feat_init, iters, stride,
+                                                          score_target=score_target)
+        elif self._shard is None or self._shard[1] == 1:
             preds, vis_e, ffeat = self._engine.refine(self, fmaps.float(), coords, feat_init, iters, stride)
         else:
             from .sharding import refine_sharded
@@ -256,7 +285,4 @@ class Pips(nn.Module):
         coord_predictions = [preds[i] for i in range(iters)]                            # :538
         last = coord_predictions[-1] if iters > 0 else start
         coord_predictions2 = [start, start] + coord_predictions + [last, last]          # :474-475, :562-563
-        losses = None
-        if return_feat:
-            return coord_predictions, coord_predictions2, vis_e, ffeat, losses
-        return coord_predictions, coord_predictions2, vis_e, losses
+        return coord_predictions, coord_predictions2, vis_e, ffeat, ce
